@@ -51,7 +51,11 @@ def parse_args():
     ap.add_argument("--max-depth", type=int, default=100)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-baseline-windows", type=int, default=0, help="windows of chunk 0 timed on the CPU (0 = all)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the token ids of the last timed step of every workload to DIR/<name>.npy (float64)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.configs is None:
         a.configs = f"{a.model}:{a.chunks_per_gpu}:{a.kv}" if a.model else DEFAULT_CONFIGS
     a.config_list = []
@@ -168,7 +172,7 @@ def run_reference(args):
     for _ in range(args.warmup):
         cpu_reference_pass(args.beam, args.max_depth, dims, w_t, sp, chunk, 1)
     times, span = [], None
-    for _ in range(max(args.steps, 1)):
+    for _ in range(args.steps):
         span, dt, nw, _ = cpu_reference_pass(args.beam, args.max_depth, dims, w_t, sp, chunk, nwin)
         times.append(dt)
     ms = 1000.0 * float(np.mean(times))
@@ -176,7 +180,7 @@ def run_reference(args):
     sample = f"{nw} of 3 reference windows of chunk 0 ({span:.2f} s of audio), greedy depth {args.max_depth}, no KV cache"
     line = {
         "impl": "reference", "metric": "audio-seconds/sec", "value": val, "unit": "audio-s/s", "n_gpus": args.gpus,
-        "steps": max(args.steps, 1), "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
+        "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": workload_name(model, chunks, args.beam, args.max_depth),
                    "path": "CPU reference-cost path (oracle port of the reference's libtorch-CPU fp32 semantics, no KV cache)",
@@ -298,12 +302,16 @@ def run_config(args, cfg, ctx):
         flush_buf.fill_(1)
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        step_e2e()
+        merged = step_e2e()
         torch.cuda.synchronize()
         e2e_ms.append(1000.0 * (time.perf_counter() - t0))
     barrier()
     gc.enable()
     steps_run = sess.last_steps()
+    outputs = None
+    if args.dump_outputs and rank == 0:   # what each timed path returned in its last step, every rank's units in global order
+        outputs = {"window_tokens": gather.as_lists(gather.np_out) if gather is not None else toks,
+                   "chunk_tokens": gather_e2e.as_lists(gather_e2e.np_out) if gather_e2e is not None else merged}
 
     def max_over_ranks(v: float) -> float:
         if world == 1:
@@ -371,7 +379,7 @@ def run_config(args, cfg, ctx):
             "rtf": (ms_step / 1000.0) / audio_s, "decode_steps_executed": steps_run,
             "e2e": {"value": e2e_val, "unit": "audio-s/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                     "ms_per_step": ms_e2e, "api": "wb_waveforms_to_tokens (windowing + batched decode + overlap merge), pinned host waveforms"},
-            "gpu_launches": launches // max(args.steps, 1), "roofline": roof,
+            "gpu_launches": launches // args.steps, "roofline": roof,
             "wall_ms_each": [round(v, 3) for v in wall_ms], "e2e_ms_each": [round(v, 3) for v in e2e_ms],
             "weights": "fp16-exact synthetic (tensor-core path)" if wh.weights_fp16_exact else "not fp16-exact: fp32 SIMT path",
             "tokens_checksum": int(sum(sum(t) for t in toks) % (1 << 31)),
@@ -379,7 +387,18 @@ def run_config(args, cfg, ctx):
         if per_rank is not None:
             res["per_rank_ms_wall_dev"] = per_rank
     sess.close()
-    return res, (dims, w_keep, sp, chunks[0], chunk_ids[0])
+    return res, (dims, w_keep, sp, chunks[0], chunk_ids[0]), outputs
+
+
+def write_outputs(out_dir, outputs: dict) -> None:
+    """One DIR/<name>.npy per token id list of lists: float64 [n, longest list], padded with -1."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, lists in outputs.items():
+        m = np.full((len(lists), max((len(t) for t in lists), default=0)), -1.0)
+        for i, t in enumerate(lists):
+            m[i, :len(t)] = t
+        np.save(d / f"{name}.npy", m)
 
 
 def run_ours(args):
@@ -403,13 +422,17 @@ def run_ours(args):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-    results, head_inputs = [], None
+    results, head_inputs, dumps = [], None, {}
     for i, cfg in enumerate(args.config_list):
-        res, inputs = run_config(args, cfg, ctx)
+        res, inputs, outputs = run_config(args, cfg, ctx)
         results.append(res)
         if i == 0:
             head_inputs = inputs
+        if outputs is not None:
+            dumps.update({f"{i}_{cfg[0]}_{cfg[1]}chunks_{cfg[2]}_{k}": v for k, v in outputs.items()})
     clocks = sampler.stop() if sampler else None
+    if dumps:
+        write_outputs(args.dump_outputs, dumps)
 
     # ---- CPU baseline beside the headline (rank 0, N=1 only)
     cpu = None

@@ -230,3 +230,21 @@ def test_bench_algorithmic_bytes_tiny_en_headline():
     assert bench.algorithmic_bytes(dims, lens, 2, 4, 100) == want == 8177565696
     # the fp16 cache halves the K/V terms only
     assert bench.algorithmic_bytes(dims, lens, 2, 2, 100) == weights * 103 + (cross * 103 + self_kv) // 2 + 100 * V * d * 2 == 6930886656
+
+
+def test_bench_dump_outputs_format_and_steps_argument(tmp_path):
+    """`bench.py --dump-outputs DIR` writes each token id list of lists as a float64 [n, longest] matrix padded with -1;
+    `--steps` below 1 is refused rather than silently raised to 1."""
+    import importlib.util
+    import subprocess
+    import sys
+    spec = importlib.util.spec_from_file_location("bench_mod", ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    bench.write_outputs(tmp_path / "out", {"0_tiny.en_1chunks_f32_window_tokens": [[50257, 50259, 7], [50257]], "empty": []})
+    m = np.load(tmp_path / "out" / "0_tiny.en_1chunks_f32_window_tokens.npy")
+    assert m.dtype == np.float64 and m.tolist() == [[50257, 50259, 7], [50257, -1, -1]]
+    assert np.load(tmp_path / "out" / "empty.npy").shape == (0, 0)
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "0"], capture_output=True, text=True,
+                       timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr
